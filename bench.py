@@ -9,6 +9,7 @@ turntable (weak scaling, no data-path collective), value = all rays of all ranks
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            our CUDA path
   python bench.py --impl reference [...]                         the reference algorithm (CPU oracle port) on host cores
+  python bench.py [...] --dump-outputs DIR                        also writes what the last timed step rendered as DIR/<name>.npy
 
 Prints ONE JSON line (rank 0).  See the prompt contract for the keys; `roofline` is for the dominant kernel (the
 field kernel: lookups + MLP), `cpu_baseline` is the oracle port timed on this box's host cores on a bounded sample.
@@ -61,7 +62,13 @@ def parse():
                     help="train mode: projected = map columns of layers 0/3 applied to the feature maps once per step (exact re-association, default); "
                          "reference = the reference's row-by-row K=703/831 input layers")
     ap.add_argument("--freeze-encoder", action="store_true", help="train mode: MLPs only (finetune mode); default trains GridEncoder inside the step")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (render_rays_test's dict, rank 0) as DIR/<name>.npy, float32; the inputs "
+                         "depend only on the arguments, so two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.mode != "frames"):
+        ap.error("--dump-outputs needs --impl ours --mode frames")
+    return args
 
 
 def peaks():
@@ -245,6 +252,7 @@ def main():
 
     import torch
     import ctypes as C
+    import numpy as np
     assert torch.cuda.is_available(), "bench.py needs a CUDA device (no CPU fallback for the product path)"
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
@@ -253,8 +261,7 @@ def main():
         import torch.distributed as dist
         dist.init_process_group("nccl", device_id=dev)
     from neo360_b200 import NeRF_TP, _lib as L, build
-    build.build()
-    lib = L.load()
+    lib = L.load(build.build())
 
     if args.mode != "frames":
         import bench_modes
@@ -300,8 +307,10 @@ def main():
 
     wh = (IMG_W, IMG_H) if (n == IMG_W * IMG_H and not os.environ.get("NEO360_NO_BLOCK_ORDER")) else None
 
+    last = {}
+
     def step_resident(s):
-        return net.render_rays_test(devrays[s % len(devrays)], chunk=CHUNK, img_wh=wh)
+        last["out"] = net.render_rays_test(devrays[s % len(devrays)], chunk=CHUNK, img_wh=wh)
 
     in_o, in_d = torch.empty(n, 3, device=dev), torch.empty(n, 3, device=dev)        # device staging of the per-step inputs
     out_rgb, out_depth = torch.empty(n, 3).pin_memory(), torch.empty(n).pin_memory()   # contiguous pinned outputs (one DMA each)
@@ -341,6 +350,12 @@ def main():
     launches = C.c_ulonglong()
     lib.neo_profile_read(None, None, C.byref(launches), None)
     net.check()
+    if args.dump_outputs and rank == 0:
+        # 11 floats per ray: a whole frame is 13.5 MB, so every array is written in full
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in last["out"].items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), t.float().cpu().numpy())
+    del last["out"]
     ms_e2e = timed(step_e2e)
     variants = {}
     if world == 1 and not args.no_extras and n == IMG_W * IMG_H:

@@ -136,12 +136,13 @@ SYMBOLS = {
 _lib = None
 
 
-def load():
-    """dlopen the in-tree library and type its entry points.  Raises if it has not been built."""
+def load(path=None):
+    """dlopen the library at `path` (default: the in-tree one) and type its entry points; the first call decides which
+    library the process uses.  Raises if it has not been built."""
     global _lib
     if _lib is not None:
         return _lib
-    path = os.environ.get("NEO360_B200_LIB") or LIB_PATH      # override: A/B runs of experimental kernel builds (tools/)
+    path = os.environ.get("NEO360_B200_LIB") or path or LIB_PATH      # override: A/B runs of experimental kernel builds (tools/)
     if not os.path.exists(path):
         raise RuntimeError(f"{path} is missing: run `python -m neo360_b200.build` (or __graft_entry__.build()); "
                            "there is no CPU fallback")

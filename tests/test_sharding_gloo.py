@@ -43,7 +43,11 @@ def _worker(rank, world, port, n, chunk, tmp):
 
 @pytest.mark.parametrize("n,chunk", [(1728, 512), (1000, 1024), (4096, 1024)])
 def test_two_rank_gloo_shard_and_gather(tmp_path, n, chunk):
+    import socket
     import torch.multiprocessing as mp
-    port = 29500 + (os.getpid() + n) % 2000
+    s = socket.socket()                  # a port the OS reports free, not a fixed one another process may hold
+    s.bind(("127.0.0.1", 0))
+    port = s.getsockname()[1]
+    s.close()
     mp.spawn(_worker, args=(2, port, n, chunk, str(tmp_path)), nprocs=2, join=True)
     assert (tmp_path / "ok0").exists() and (tmp_path / "ok1").exists()

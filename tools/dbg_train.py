@@ -1,4 +1,6 @@
-import sys; sys.path.insert(0,'/root/repo'); sys.path.insert(0,'/root/repo/tests')
+import os, sys
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tests'))
 import torch
 from test_training import _tiny, md
 from neo360_b200 import training, synth
