@@ -175,21 +175,30 @@ def piecewise_constant_pdf(bins: Tensor, w: Tensor, m: int, u_rand: Optional[Ten
     return b0 + tau * (b1 - b0)
 
 
+def fg_points(o, d, t):
+    """fg sample points o + t d for t (B,N) (helper.py:52-53)."""
+    return o[:, None, :] + t[..., None] * d[:, None, :]
+
+
+def bg_points(o, d, s, far, far_unc=3.0):
+    """bg points for inverse radii s (B,N): the unit-sphere points fed to the encoding and the lookup points
+    o + (far (1-s) + far_unc s) d (quirk Q2)."""
+    t_lin = far * (1.0 - s) + far_unc * s
+    return depth2pts_outside(o, d, s), o[:, None, :] + t_lin[..., None] * d[:, None, :]
+
+
 def resample_fg(o, d, t_old, w, m, u_rand=None):
     mids = 0.5 * (t_old[..., 1:] + t_old[..., :-1])
     t_new = piecewise_constant_pdf(mids, w[..., 1:-1], m, u_rand).detach()      # helper.py:222-224: no gradient through the new samples
     t = torch.sort(torch.cat([t_old, t_new], -1), -1).values
-    return t, o[:, None, :] + t[..., None] * d[:, None, :]
+    return t, fg_points(o, d, t)
 
 
 def resample_bg(o, d, s_old, w, m, far, far_unc=3.0, u_rand=None):
     mids = 0.5 * (s_old[..., 1:] + s_old[..., :-1])
     s_new = piecewise_constant_pdf(mids, w[..., 1:-1], m, u_rand).detach()      # helper.py:222-224
-    s = torch.sort(torch.cat([s_old, s_new], -1), -1).values
-    t_lin = far * (1.0 - s) + far_unc * s
-    s = torch.flip(s, dims=[-1])
-    t_lin = torch.flip(t_lin, dims=[-1])
-    return s, depth2pts_outside(o, d, s), o[:, None, :] + t_lin[..., None] * d[:, None, :]
+    s = torch.flip(torch.sort(torch.cat([s_old, s_new], -1), -1).values, dims=[-1])
+    return (s, *bg_points(o, d, s, far, far_unc))
 
 
 # --------------------------------------------------------------------------------------------
@@ -223,25 +232,30 @@ def bilinear_zeros(fmap: Tensor, gx: Tensor, gy: Tensor, impl: str = "explicit")
         g = torch.stack([gx, gy], -1)[:, :, None, :]
         return F.grid_sample(fmap, g, mode="bilinear", padding_mode="zeros", align_corners=True)[..., 0] \
             .permute(0, 2, 1)
+    x0, y0, w = bilinear_quad(gx, gy, H, W)
+    flat = fmap.reshape(NV, C, H * W).permute(0, 2, 1)  # (NV, HW, C)
+
+    def tap(xx, yy, ww):
+        idx = (yy.clamp(0, H - 1) * W + xx.clamp(0, W - 1)).long()
+        val = torch.gather(flat, 1, idx[..., None].expand(-1, -1, C))
+        return val * ww[..., None]
+
+    return tap(x0, y0, w[..., 0]) + tap(x0 + 1, y0, w[..., 1]) + tap(x0, y0 + 1, w[..., 2]) + tap(x0 + 1, y0 + 1, w[..., 3])
+
+
+def bilinear_quad(gx: Tensor, gy: Tensor, H: int, W: int):
+    """The 2x2 tap quad of grid_sample(bilinear, align_corners=True, zeros): base texel (x0, y0) (floats, unclamped) and the
+    weights (..., 4) of nw, ne, sw, se, zero for a tap outside the map."""
     ix = ((gx + 1) / 2) * (W - 1)
     iy = ((gy + 1) / 2) * (H - 1)
     x0 = torch.floor(ix)
     y0 = torch.floor(iy)
     x1 = x0 + 1
     y1 = y0 + 1
-    w_nw = (x1 - ix) * (y1 - iy)
-    w_ne = (ix - x0) * (y1 - iy)
-    w_sw = (x1 - ix) * (iy - y0)
-    w_se = (ix - x0) * (iy - y0)
-    flat = fmap.reshape(NV, C, H * W).permute(0, 2, 1)  # (NV, HW, C)
-
-    def tap(xx, yy, ww):
-        ok = (xx >= 0) & (xx <= W - 1) & (yy >= 0) & (yy <= H - 1)
-        idx = (yy.clamp(0, H - 1) * W + xx.clamp(0, W - 1)).long()
-        val = torch.gather(flat, 1, idx[..., None].expand(-1, -1, C))
-        return val * (ww * ok)[..., None]
-
-    return tap(x0, y0, w_nw) + tap(x1, y0, w_ne) + tap(x0, y1, w_sw) + tap(x1, y1, w_se)
+    ok = lambda xx, yy: (xx >= 0) & (xx <= W - 1) & (yy >= 0) & (yy <= H - 1)
+    w = torch.stack([(x1 - ix) * (y1 - iy) * ok(x0, y0), (ix - x0) * (y1 - iy) * ok(x1, y0),
+                     (x1 - ix) * (iy - y0) * ok(x0, y1), (ix - x0) * (iy - y0) * ok(x1, y1)], -1)
+    return x0, y0, w
 
 
 @dataclass
@@ -268,6 +282,12 @@ def triplane_lookup(p_cam: Tensor, sc: Scene, impl="explicit") -> Tensor:
 
 def local_lookup(p_cam: Tensor, sc: Scene, impl="explicit") -> Tensor:
     """get_local_feats (model.py:239-264) -> projection (util.py:92-111) -> index (encoder_pn.py:101-152)."""
+    gx, gy = local_coords(p_cam, sc)
+    return bilinear_zeros(sc.latent, gx, gy, impl)
+
+
+def local_coords(p_cam: Tensor, sc: Scene):
+    """Grid coordinates of the camera-frame points in the pixel-aligned latent (util.py:92-111, encoder_pn.py:116-120)."""
     uv = -p_cam[..., :2] / (p_cam[..., 2:] + 1e-9)
     dev = p_cam.device
     uv = uv * torch.tensor([sc.focal, -sc.focal], device=dev) + torch.tensor([sc.cx, sc.cy], device=dev)
@@ -276,7 +296,7 @@ def local_lookup(p_cam: Tensor, sc: Scene, impl="explicit") -> Tensor:
     ls = ls / (ls - 1) * 2.0
     scale = ls / torch.tensor([float(sc.img_w), float(sc.img_h)], device=dev)
     uv = uv * scale - 1.0
-    return bilinear_zeros(sc.latent, uv[..., 0], uv[..., 1], impl)
+    return uv[..., 0], uv[..., 1]
 
 
 # --------------------------------------------------------------------------------------------
@@ -318,11 +338,17 @@ def field(P, pre, pts_cam_enc_in: Tensor, dirs_cam: Tensor, world, local, B: int
     encoding is tiled along the RAY axis, so row j=b*N+s sees ray (j mod B)."""
     enc = pos_enc(pts_cam_enc_in, 0, 10)
     denc = pos_enc(dirs_cam, 0, 4)                       # (NV,B,27)
-    dir_tile = denc[:, None].repeat(1, 1, N, 1).reshape(-1, denc.shape[-1])
+    dir_tile = q1_dir_tile(denc, N)
     raw_rgb, raw_sigma = mlp_forward(P, pre, enc, dir_tile, world, local, nv)
     sigma = F.softplus(raw_sigma.reshape(B, N, 1) - 1.0)
     rgb = torch.sigmoid(raw_rgb.reshape(B, N, 3)) * (1 + 2 * 0.001) - 0.001
     return rgb, sigma
+
+
+def q1_dir_tile(denc: Tensor, N: int) -> Tensor:
+    """(NV,B,C) -> (NV*B*N, C): the reference tiles the direction encoding along the RAY axis (model.py:357-360), so row
+    j = b*N+s of each view is conditioned on ray (j mod B) of the batch (quirk Q1)."""
+    return denc[:, None].repeat(1, 1, N, 1).reshape(-1, denc.shape[-1])
 
 
 # --------------------------------------------------------------------------------------------

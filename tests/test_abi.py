@@ -102,3 +102,20 @@ def test_blocked_frame_order_is_a_block_permutation(wh):
         assert torch.equal(y - y[:, :1], torch.arange(32).div(8, rounding_mode="floor").expand_as(y))
         assert torch.equal(x - x[:, :1], (torch.arange(32) % 8).expand_as(x))
         assert bool((x[:, 0] % 8 == 0).all()) and bool((y[:, 0] % 4 == 0).all())
+
+
+@pytest.mark.parametrize("nv,hw,code", [(9, (24, 32), -5), (3, (1, 32), -1), (3, (32, 1), -1)])
+def test_scene_create_refusals_without_gpu(lib, nv, hw, code):
+    """neo_scene_create refuses more source views than the TC kernel's kMaxViews = 8 (NEO_ERR_UNSUPPORTED) and a 1 x k feature map
+    (NEO_ERR_INVALID: grid_sample's align_corners scaling divides by size - 1) before it touches the device."""
+    from neo360_b200 import _lib as L
+    d = L.NeoSceneDesc()
+    d.nv, d.world_ch, d.local_ch = nv, 128, 512
+    d.plane_h, d.plane_w = hw
+    d.lat_h, d.lat_w = 24, 32
+    d.img_w, d.img_h = 64, 48
+    mlps = (L.NeoMLPParams * 4)()
+    h = C.c_void_p()
+    assert lib.neo_scene_create(C.byref(d), mlps, 3, C.byref(h), None) == code
+    assert not h.value
+    assert (b"views" if nv > 8 else b"2x2") in lib.neo_last_error()
